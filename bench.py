@@ -60,7 +60,23 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the sustained / graph / C2-query legs (profiling runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result of the last timed step as DIR/<name>.npy (float64), to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        # the reference arm's sample is sized by the host's core count, so its inputs are not the same from machine to machine
+        ap.error("--dump-outputs needs --impl b200")
+    return args
+
+
+def dump_outputs(out_dir, res):
+    """The arrays a caller of the timed path receives (capi.Result), as float64 .npy files.  The int64 columns of this
+    query are row numbers, counts and group ids, far below 2**53, so the conversion is exact."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name in ("group_id", "rows", "is_float", "val_i64", "val_f64"):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(getattr(res, name), dtype=np.float64))
 
 
 def load_pkg():
@@ -461,6 +477,8 @@ def main():
     except Exception as ex:  # noqa: BLE001 -- keep the bench line alive: the plain call is then the timed one
         graph_note = {"error": str(ex)[:200]}
         dt, last, timed_step = d_plain, last_plain, step
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     kernel_timing = "cuda events inside the plain calls of the same step (a graph replay has no per-kernel events); value is timed on the prepared-query path"
     rows_step = stats_acc[-1].rows_scanned
     scan_ms = float(np.mean([s.scan_kernel_ms for s in stats_acc]))

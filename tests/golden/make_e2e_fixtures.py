@@ -1,20 +1,18 @@
 #!/usr/bin/env python
 """Generates tests/golden/e2e_cases.json from the reference's own end-to-end measure cases
-(/root/reference/test/cases/measure/data/{input,want,testdata} + pkg/test/measure/testdata/measures): the data points
+(<banyandb>/test/cases/measure/data/{input,want,testdata} + pkg/test/measure/testdata/measures): the data points
 the integration suite writes, the query of each case and the rows it expects.  Only cases inside the hot path are
-taken (group-by + aggregation, optional Top / tag filter).  Run in the build container (the reference tree is not
-on the GPU box); the JSON it writes is the committed fixture.
+taken (group-by + aggregation, optional Top / tag filter).  The JSON it writes is the committed fixture, so the
+tests need no checkout of BanyanDB.
 
-    python tests/golden/make_e2e_fixtures.py
+    python tests/golden/make_e2e_fixtures.py <banyandb checkout>
 """
 import json
 import os
+import sys
 
 import yaml
 
-REF = "/root/reference"
-DATA = os.path.join(REF, "test/cases/measure/data")
-SCHEMAS = os.path.join(REF, "pkg/test/measure/testdata/measures")
 # case -> data file written by test/cases/init.go:88,105 for that measure (group sw_metric)
 CASES = {
     "float_top_mean": "service_instance_float_metric_data.json",
@@ -55,15 +53,18 @@ def scalar(v):
 
 
 def main():
+    ref = sys.argv[1]
+    data_dir = os.path.join(ref, "test/cases/measure/data")
+    schemas = os.path.join(ref, "pkg/test/measure/testdata/measures")
     out = {}
     for case, data_file in CASES.items():
-        q = yaml.safe_load(open(os.path.join(DATA, "input", case + ".yaml")))
-        want = yaml.safe_load(open(os.path.join(DATA, "want", case + ".yaml")))
-        schema = json.load(open(os.path.join(SCHEMAS, q["name"] + ".json")))
+        q = yaml.safe_load(open(os.path.join(data_dir, "input", case + ".yaml")))
+        want = yaml.safe_load(open(os.path.join(data_dir, "want", case + ".yaml")))
+        schema = json.load(open(os.path.join(schemas, q["name"] + ".json")))
         tags = [t["name"] for t in schema["tag_families"][0]["tags"]]
         fields = [(f["name"], f["field_type"]) for f in schema["fields"]]
         rows = []
-        for dp in json.load(open(os.path.join(DATA, "testdata", data_file))):
+        for dp in json.load(open(os.path.join(data_dir, "testdata", data_file))):
             tv = [scalar(t)["value"] for t in dp["tag_families"][0]["tags"]]
             fv = [scalar(f) for f in dp["fields"]]
             rows.append({"tags": tv, "fields": [f["value"] for f in fv]})
