@@ -200,8 +200,8 @@ int bydb_scan_agg(bydb_ctx *ctx, const bydb_query *q, bydb_result *out);
  * BYDB_ENOTSUP, more than max_values distinct values over the selected blocks BYDB_ENOMEM (the reference's aggregation
  * memory budget), a value longer than 64 bytes BYDB_ENOTSUP.  Device side: one pass collects the distinct values from the
  * dictionary pages, then ONE SCAN PASS PER VALUE (the key as an extra predicate) fills that value's slice of a composite
- * partial table; stats count every pass.  Not available through the prepared / partial-table / multi-GPU entry points,
- * and not over parts that overlap in time. */
+ * partial table; stats count every pass.  Across GPUs: bydb_scan_reduce_keyed below.  Not available through the prepared /
+ * partial-table / host-image entry points, and not over parts that overlap in time. */
 typedef struct {
     const char *family;    /* tag family of the key tag                                      */
     const char *tag;       /* tag name                                                       */
@@ -347,6 +347,27 @@ int bydb_scan_reduce_prepared(bydb_ctx *ctx, bydb_prepared *pq, int32_t root, by
  * the duration of the call (with BYDB_Q_HOST_ZERO_COPY only the block directory is uploaded and the scan pulls the pages it
  * touches over PCIe), scanned into the root's mailbox, dropped.  q->parts / q->n_parts are ignored. */
 int bydb_scan_reduce_host(bydb_ctx *ctx, uint32_t n_parts, const bydb_part_files *parts, const bydb_query *q, int32_t root, bydb_result *out);
+
+/* Group-by on a stored tag as a collective (bydb_scan_agg_keyed across the connected ranks): the root gets exactly what ONE
+ * context scanning every rank's parts and series would return from bydb_scan_agg_keyed -- the same rows in the same order
+ * (insertion order, or Top-N rank order with ties to the group inserted first), the same key bytes and series group per row,
+ * int64 results, counts, min and max bit-identical; float sums add the ranks in rank order (within 1e-12 relative of the
+ * single-context sum).  Key ids index the root's key table, which numbers the values in order of first occurrence over
+ * (rank, that rank's own value order).  Every rank passes the same series-group count, aggregations, Top-N, key and
+ * max_values; q names THIS rank's parts and series.  A series may live on several ranks only in pieces that do not overlap in
+ * time (the duplicate rule of bydb_scan_reduce).  The other ranks get n_rows = 0, n_keys = 0 and their own scan statistics.
+ * Each rank finds its own distinct values, runs one scan pass per value into its slot of the root's mailbox and leaves there its
+ * dictionary and where each composite group first showed; the root unites the dictionaries, folds the slices in rank order and
+ * restores the insertion order on the device.  Epochs, slot parities and waits are bydb_scan_reduce's: keyed and plain
+ * collectives may alternate on the same mailboxes, and a failure on any rank leaves them usable.  Errors: a rank's own failure
+ * (BYDB_ENOTSUP for a plain-encoded key block or a value over 64 bytes, BYDB_EINVAL for a key tag that is not a string / binary
+ * dictionary tag or a slot too small for the table, BYDB_ENOMEM for more than max_values values on that rank, BYDB_ENOTSUP for
+ * parts of that rank that overlap in time) is returned by that rank and by the root; more than max_values distinct values over
+ * all ranks is BYDB_ENOMEM on the root.
+ * bydb_keyed_reduce_layout (host only) gives the slot size such a query needs: pass the largest over the queries to come (and
+ * over bydb_partials_layout().total_bytes of the plain collectives) as max_table_bytes of bydb_comm_export. */
+int bydb_keyed_reduce_layout(const bydb_query *q, const bydb_group_key *key, uint64_t *slot_bytes);
+int bydb_scan_reduce_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key *key, int32_t root, bydb_keyed_result *out);
 
 const char *bydb_last_error(void);
 const char *bydb_version(void);

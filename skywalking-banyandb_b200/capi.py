@@ -105,6 +105,7 @@ EXPORTS = ["bydb_init", "bydb_shutdown", "bydb_part_register", "bydb_part_releas
            "bydb_query_release", "bydb_partials_layout",
            "bydb_scan_partials", "bydb_partials_combine", "bydb_reduce_finalize", "bydb_partials_rows", "bydb_partial_rows_free", "bydb_comm_export", "bydb_comm_connect",
            "bydb_scan_reduce", "bydb_scan_reduce_prepared", "bydb_scan_reduce_host", "bydb_scan_agg_keyed", "bydb_keyed_result_free",
+           "bydb_keyed_reduce_layout", "bydb_scan_reduce_keyed",
            "bydb_encode_pages", "bydb_encoded_pages_free", "bydb_last_error", "bydb_version"]
 
 _lib = None
@@ -140,6 +141,8 @@ def load_library():
     L.bydb_scan_agg_keyed.argtypes = [C.c_void_p, C.POINTER(_Query), C.POINTER(_GroupKey), C.POINTER(_KeyedResult)]
     L.bydb_keyed_result_free.argtypes = [C.c_void_p, C.POINTER(_KeyedResult)]
     L.bydb_keyed_result_free.restype = None
+    L.bydb_keyed_reduce_layout.argtypes = [C.POINTER(_Query), C.POINTER(_GroupKey), C.POINTER(C.c_uint64)]
+    L.bydb_scan_reduce_keyed.argtypes = [C.c_void_p, C.POINTER(_Query), C.POINTER(_GroupKey), C.c_int32, C.POINTER(_KeyedResult)]
     L.bydb_encode_pages.argtypes = [C.c_void_p, C.POINTER(_EncodeInput), C.POINTER(_EncodedPages)]
     L.bydb_encoded_pages_free.argtypes = [C.c_void_p, C.POINTER(_EncodedPages)]
     L.bydb_encoded_pages_free.restype = None
@@ -303,6 +306,16 @@ def _mk_query(q: Query, keep: list) -> _Query:
     return cq
 
 
+def keyed_reduce_layout(q: Query, family: str, tag: str, max_values: int = 0) -> int:
+    """Mailbox slot bytes the keyed collective needs for q (bydb_keyed_reduce_layout; host only, no device)."""
+    keep: list = []
+    cq = _mk_query(q, keep)
+    gk = _GroupKey(family.encode(), tag.encode(), max_values, 0)
+    out = C.c_uint64(0)
+    _check(load_library().bydb_keyed_reduce_layout(C.byref(cq), C.byref(gk), C.byref(out)))
+    return out.value
+
+
 class PreparedQuery:
     """A Query marshalled once into the C struct (with everything it points at kept alive): repeated calls skip
     the per-call ctypes work.  Context methods take a Query or a PreparedQuery."""
@@ -438,9 +451,12 @@ class Context:
         gk = _GroupKey(fb, tb, max_values, 0)
         r = _KeyedResult()
         _check(self._L.bydb_scan_agg_keyed(self._h, C.byref(cq), C.byref(gk), C.byref(r)))
+        return self._read_keyed(r, len(q.aggs))
+
+    def _read_keyed(self, r: _KeyedResult, n_aggs: int) -> Result:
         try:
             if r.base.n_rows == 0 and not r.base.owner:
-                a = len(q.aggs)
+                a = n_aggs
                 res = Result(np.zeros(0, np.int32), np.zeros(0, np.int64), np.zeros(a, bool), np.zeros((0, a), np.int64),
                              np.zeros((0, a), np.float64), Stats.of(r.base.stats))
             else:
@@ -549,6 +565,20 @@ class Context:
             return _read_result(r)
         finally:
             self._L.bydb_result_free(self._h, C.byref(r))
+
+    def keyed_reduce_layout(self, q: Query, family: str, tag: str, max_values: int = 0) -> int:
+        """Mailbox slot bytes scan_reduce_keyed needs for q: pass the largest over the queries to come to comm_export."""
+        return keyed_reduce_layout(q, family, tag, max_values)
+
+    def scan_reduce_keyed(self, q: Query, family: str, tag: str, root: int = 0, max_values: int = 0) -> Result:
+        """Group-by on a stored tag as a collective (bydb_scan_reduce_keyed): the root gets what scan_agg_keyed over every rank's
+        parts and series returns, .key and .n_keys included; the other ranks get an empty result with their own scan statistics."""
+        keep: list = []
+        cq = _mk_query(q, keep)
+        gk = _GroupKey(family.encode(), tag.encode(), max_values, 0)
+        r = _KeyedResult()
+        _check(self._L.bydb_scan_reduce_keyed(self._h, C.byref(cq), C.byref(gk), root, C.byref(r)))
+        return self._read_keyed(r, len(q.aggs))
 
     def scan_reduce_host(self, parts: Sequence[Dict[str, Union[bytes, np.ndarray]]], q: Query, root: int = 0) -> Result:
         keep: list = []

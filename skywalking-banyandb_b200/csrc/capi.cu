@@ -1598,24 +1598,16 @@ struct KeyedOwner {
     std::vector<uint32_t> key_off;
     std::vector<uint8_t> key_bytes;
 };
-}  // namespace
 
-void bydb_keyed_result_free(bydb_ctx *ctx, bydb_keyed_result *r);
-void bydb_encoded_pages_free(bydb_ctx *ctx, bydb_encoded_pages *r);
-
-// Group-by on a stored tag (per-row key): see "Group key" in scan_kernels.cu for the device side.
-int bydb_scan_agg_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key *key, bydb_keyed_result *out) {
-    return guarded([&]() -> int {
-    if (!ctx || !out) return fail(BYDB_EINVAL, "ctx/out is NULL");
-    memset(out, 0, sizeof *out);
+// The checks every group-key entry point makes before it touches the device: the key, its value cap, the predicate budget,
+// the plan, and no two parts that overlap in time.
+int keyed_prepare(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key *key, Plan &plan, uint32_t &cap) {
     int rc = validate_query(q, true);
     if (rc) return rc;
     if (!key || !key->family || !key->tag) return fail(BYDB_EINVAL, "group key without family/tag");
-    const uint32_t cap = key->max_values ? key->max_values : 64u;
+    cap = key->max_values ? key->max_values : 64u;
     if (cap > kMaxKeyValues) return fail(BYDB_EINVAL, "bydb_group_key.max_values above 256");
     if (q->n_preds + 1 > kMaxPreds) return fail(BYDB_ENOTSUP, "a group-key query takes at most 7 predicates");
-    g_last_dev_err = 0;
-    Plan plan;
     rc = make_plan(ctx, q, nullptr, plan);
     if (rc) return rc;
     for (size_t a = 0; a < plan.parts.size(); ++a)
@@ -1625,15 +1617,23 @@ int bydb_scan_agg_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key
             if (std::max(std::max(x.min_ts, y.min_ts), q->tmin) <= std::min(std::min(x.max_ts, y.max_ts), q->tmax))
                 return fail(BYDB_ENOTSUP, "group-key query over parts that overlap in time (version dedup) is not supported on the device path");
         }
-    CUDA_TRY(cudaSetDevice(ctx->device));
-    SlotLease lease(ctx);
-    if (lease.init()) return fail(BYDB_EIO, "cannot create stream");
-    ExecSlot &slot = *lease.slot;
-    cudaStream_t stream = slot.stream;
-    const size_t F = plan.fcols.size(), NS = q->n_series, NB = plan.total_blocks, G = static_cast<size_t>(plan.n_groups);
-    memset(&out->base.stats, 0, sizeof out->base.stats);
+    return 0;
+}
 
-    // ---- 1. the distinct key values of the selected blocks
+// Step 1 of a group-key query: the distinct key values of the selected blocks.  The device copies stay in `sc`: the query's
+// series ids at d_sids, the packed values (cap x kMaxLit bytes) at d_vals, their lengths at d_lens.
+struct KeyValues {
+    Scratch sc;
+    const uint64_t *d_sids = nullptr;
+    const uint8_t *d_vals = nullptr;
+    const uint32_t *d_lens = nullptr;
+    std::vector<std::vector<uint8_t>> values;
+};
+
+int keyed_values(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key *key, uint32_t cap, const Plan &plan, ExecSlot &slot, bydb_stats *stats,
+                 KeyValues &kv) {
+    cudaStream_t stream = slot.stream;
+    const size_t NS = q->n_series, NB = plan.total_blocks;
     size_t o = 0;
     auto carve = [&](size_t bytes) {
         size_t at = o;
@@ -1643,9 +1643,12 @@ int bydb_scan_agg_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key
     const size_t a_sids = carve(NS * 8), a_slots = carve(kKeySlots * 8), a_ctl = carve(16), a_vals = carve(static_cast<size_t>(cap) * kMaxLit),
                  a_lens = carve(static_cast<size_t>(cap) * 4);
     const size_t a_total = o;
-    Scratch ka;
+    Scratch &ka = kv.sc;
     ka.stream = stream;
     CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&ka.base), a_total, stream));
+    kv.d_sids = reinterpret_cast<const uint64_t *>(ka.base + a_sids);
+    kv.d_vals = ka.base + a_vals;
+    kv.d_lens = reinterpret_cast<const uint32_t *>(ka.base + a_lens);
     const size_t back_bytes = a_total - a_ctl;  // ctl | vals | lens come back in one copy
     if (slot.ensure_pinned(std::max(back_bytes, NS * 8) + 256)) return fail(BYDB_ENOMEM, "cudaMallocHost failed");
     if (NS) memcpy(slot.pinned, q->series_ids, NS * 8);
@@ -1684,9 +1687,9 @@ int bydb_scan_agg_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key
     CUDA_TRY(cudaMemcpyAsync(slot.pinned, ka.base + a_ctl, back_bytes, cudaMemcpyDeviceToHost, stream));
     CUDA_TRY(cudaStreamSynchronize(stream));
     CUDA_TRY(cudaGetLastError());
-    out->base.stats.kernel_launches += 2;
-    out->base.stats.h2d_bytes += NS * 8;
-    out->base.stats.d2h_bytes += back_bytes;
+    stats->kernel_launches += 2;
+    stats->h2d_bytes += NS * 8;
+    stats->d2h_bytes += back_bytes;
     const uint32_t *ctl = reinterpret_cast<const uint32_t *>(slot.pinned);
     if (ctl[1] != 0) {
         g_last_dev_err = ctl[1];
@@ -1695,12 +1698,127 @@ int bydb_scan_agg_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key
         return fail(dev_err_code(ctl[1]), std::string(dev_err_text(ctl[1])) + buf);
     }
     const size_t V = std::min<size_t>(ctl[0], cap);
-    std::vector<std::vector<uint8_t>> values(V);
-    {
-        const uint8_t *hv = slot.pinned + (a_vals - a_ctl);
-        const uint32_t *hl = reinterpret_cast<const uint32_t *>(slot.pinned + (a_lens - a_ctl));
-        for (size_t v = 0; v < V; ++v) values[v].assign(hv + v * kMaxLit, hv + v * kMaxLit + hl[v]);
+    kv.values.assign(V, {});
+    const uint8_t *hv = slot.pinned + (a_vals - a_ctl);
+    const uint32_t *hl = reinterpret_cast<const uint32_t *>(slot.pinned + (a_lens - a_ctl));
+    for (size_t v = 0; v < V; ++v) kv.values[v].assign(hv + v * kMaxLit, hv + v * kMaxLit + hl[v]);
+    return 0;
+}
+
+// Step 2: one scan pass per value v (the key as an extra predicate) into slice v of a composite table of V x G groups
+// (value-major) at `table` with layout `tl`; pass v leaves its column types at coltype[v * F] and, per series, where it first
+// shows v at kts / krow[v * NS].  Every pass is synchronised and its device errors collected.
+int keyed_passes(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key *key, Plan &plan, ExecSlot &slot, const KeyValues &kv, uint8_t *table,
+                 const TableLayout &tl, int64_t *coltype, int64_t *kts, uint32_t *krow, bydb_stats *stats) {
+    cudaStream_t stream = slot.stream;
+    const size_t F = plan.fcols.size(), NS = q->n_series, G = static_cast<size_t>(plan.n_groups);
+    std::vector<bydb_pred> preds(q->preds, q->preds + q->n_preds);
+    preds.emplace_back();
+    bydb_query qv = *q;
+    qv.n_preds = q->n_preds + 1;
+    for (size_t v = 0; v < kv.values.size(); ++v) {
+        bydb_pred &kpred = preds.back();
+        memset(&kpred, 0, sizeof kpred);
+        kpred.family = key->family;
+        kpred.tag = key->tag;
+        kpred.op = kv.values[v].empty() ? kOpEqOrNil : BYDB_OP_EQ;  // a nil cell and "" are the same key (groupby.go:226-254)
+        kpred.value_type = BYDB_VT_STR;
+        kpred.lit = kv.values[v].data();
+        kpred.lit_len = kv.values[v].size();
+        qv.preds = preds.data();
+        KeyedPass pass;
+        pass.group_off = v * G;
+        pass.coltype = coltype + v * F;
+        pass.kts = kts + v * NS;
+        pass.krow = krow + v * NS;
+        int rc = run_scan(ctx, &qv, plan, slot, stream, table, tl, stats, 0, true, &pass);
+        cudaError_t ce = cudaStreamSynchronize(stream);  // also on failure: nothing may be in flight when the slot goes back
+        if (!rc && ce != cudaSuccess) rc = fail(BYDB_EIO, cudaGetErrorString(ce));
+        if (!rc) rc = collect_scan(slot, stats);
+        if (rc) return rc;
     }
+    return 0;
+}
+
+// order | group_start of the series groups (run_scan's copies live in its own scratch), uploaded into `sc` through the staging
+int upload_group_order(const bydb_query *q, size_t G, ExecSlot &slot, Scratch &sc, const int32_t **order_out, const int32_t **gstart_out) {
+    const size_t NS = q->n_series;
+    std::vector<int32_t> order(NS), gstart(G + 1, 0);
+    if (q->series_group) {
+        for (size_t i = 0; i < NS; ++i) gstart[static_cast<size_t>(q->series_group[i]) + 1]++;
+        for (size_t g = 0; g < G; ++g) gstart[g + 1] += gstart[g];
+        std::vector<int32_t> cur(gstart.begin(), gstart.end() - 1);
+        for (size_t i = 0; i < NS; ++i) order[cur[q->series_group[i]]++] = static_cast<int32_t>(i);
+    } else {
+        for (size_t i = 0; i < NS; ++i) order[i] = static_cast<int32_t>(i);
+        gstart[1] = static_cast<int32_t>(NS);
+    }
+    sc.stream = slot.stream;
+    const size_t c_gstart = align_up(NS * 4, 256);
+    CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&sc.base), c_gstart + (G + 1) * 4, slot.stream));
+    if (NS) memcpy(slot.pinned, order.data(), NS * 4);
+    memcpy(slot.pinned + c_gstart, gstart.data(), (G + 1) * 4);
+    CUDA_TRY(cudaMemcpyAsync(sc.base, slot.pinned, c_gstart + (G + 1) * 4, cudaMemcpyHostToDevice, slot.stream));
+    *order_out = reinterpret_cast<const int32_t *>(sc.base);
+    *gstart_out = reinterpret_cast<const int32_t *>(sc.base + c_gstart);
+    return 0;
+}
+
+TablePtrs table_ptrs(uint8_t *t, const TableLayout &tl) {
+    TablePtrs tp;
+    tp.sum_f64 = reinterpret_cast<double *>(t + tl.off_sum_f64);
+    tp.max_f64 = reinterpret_cast<double *>(t + tl.off_max_f64);
+    tp.negmin_f64 = reinterpret_cast<double *>(t + tl.off_negmin_f64);
+    tp.sum_i64 = reinterpret_cast<int64_t *>(t + tl.off_sum_i64);
+    tp.cnt = reinterpret_cast<int64_t *>(t + tl.off_cnt);
+    tp.rows = reinterpret_cast<int64_t *>(t + tl.off_rows);
+    tp.max_i64 = reinterpret_cast<int64_t *>(t + tl.off_max_i64);
+    tp.notmin_i64 = reinterpret_cast<int64_t *>(t + tl.off_notmin_i64);
+    tp.coltype = reinterpret_cast<int64_t *>(t + tl.off_coltype);
+    return tp;
+}
+
+// The finalised rows carry the position of their composite group in insertion order: back to (group of the series, key value)
+void keyed_split_rows(bydb_keyed_result *out, const std::vector<int32_t> &perm, size_t G) {
+    auto *owner = static_cast<KeyedOwner *>(out->owner);
+    auto *ro = static_cast<ResultOwner *>(out->base.owner);
+    owner->key_id.resize(ro->group_id.size());
+    for (size_t r = 0; r < ro->group_id.size(); ++r) {
+        const int32_t comp = perm[static_cast<size_t>(ro->group_id[r])];
+        owner->key_id[r] = comp / static_cast<int32_t>(G);
+        ro->group_id[r] = comp % static_cast<int32_t>(G);
+    }
+    out->key_id = owner->key_id.data();
+}
+}  // namespace
+
+void bydb_keyed_result_free(bydb_ctx *ctx, bydb_keyed_result *r);
+void bydb_encoded_pages_free(bydb_ctx *ctx, bydb_encoded_pages *r);
+
+// Group-by on a stored tag (per-row key): see "Group key" in scan_kernels.cu for the device side.
+int bydb_scan_agg_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key *key, bydb_keyed_result *out) {
+    return guarded([&]() -> int {
+    if (!ctx || !out) return fail(BYDB_EINVAL, "ctx/out is NULL");
+    memset(out, 0, sizeof *out);
+    Plan plan;
+    uint32_t cap = 0;
+    int rc = keyed_prepare(ctx, q, key, plan, cap);
+    if (rc) return rc;
+    g_last_dev_err = 0;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    SlotLease lease(ctx);
+    if (lease.init()) return fail(BYDB_EIO, "cannot create stream");
+    ExecSlot &slot = *lease.slot;
+    cudaStream_t stream = slot.stream;
+    const size_t F = plan.fcols.size(), NS = q->n_series, G = static_cast<size_t>(plan.n_groups);
+    memset(&out->base.stats, 0, sizeof out->base.stats);
+
+    // ---- 1. the distinct key values of the selected blocks
+    KeyValues kv;
+    rc = keyed_values(ctx, q, key, cap, plan, slot, &out->base.stats, kv);
+    if (rc) return rc;
+    const std::vector<std::vector<uint8_t>> &values = kv.values;
+    const size_t V = values.size();
     auto owner = new KeyedOwner();
     out->owner = owner;
     bool done = false;
@@ -1730,7 +1848,12 @@ int bydb_scan_agg_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key
     const size_t GP = G * V;
     if (GP > 0x7fffffffull / std::max<size_t>(F, 1)) return fail(BYDB_ENOMEM, "group-key query: too many composite groups");
     TableLayout tlc(GP, F);
-    o = 0;
+    size_t o = 0;
+    auto carve = [&](size_t bytes) {
+        size_t at = o;
+        o = align_up(o + bytes, 256);
+        return at;
+    };
     const size_t b_src = carve(tlc.total), b_dst = carve(tlc.total), b_ct = carve(V * F * 8), b_kts = carve(V * NS * 8), b_krow = carve(V * NS * 4),
                  b_slot = carve(NS * V * 4), b_first = carve(GP * 4), b_perm = carve(GP * 4), b_np = carve(16);
     Scratch kb;
@@ -1742,31 +1865,9 @@ int bydb_scan_agg_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key
         const size_t A = q->n_aggs;
         if (slot.ensure_pinned(NS * 12 + (G + 1) * 4 + GP * (12 + 16 * A) + 16 * A + 8192)) return fail(BYDB_ENOMEM, "cudaMallocHost failed");
     }
-    std::vector<bydb_pred> preds(q->preds, q->preds + q->n_preds);
-    preds.emplace_back();
-    bydb_query qv = *q;
-    qv.n_preds = q->n_preds + 1;
-    for (size_t v = 0; v < V; ++v) {
-        bydb_pred &kpred = preds.back();
-        memset(&kpred, 0, sizeof kpred);
-        kpred.family = key->family;
-        kpred.tag = key->tag;
-        kpred.op = values[v].empty() ? kOpEqOrNil : BYDB_OP_EQ;  // a nil cell and "" are the same key (groupby.go:226-254)
-        kpred.value_type = BYDB_VT_STR;
-        kpred.lit = values[v].data();
-        kpred.lit_len = values[v].size();
-        qv.preds = preds.data();
-        KeyedPass pass;
-        pass.group_off = v * G;
-        pass.coltype = reinterpret_cast<int64_t *>(kb.base + b_ct) + v * F;
-        pass.kts = reinterpret_cast<int64_t *>(kb.base + b_kts) + v * NS;
-        pass.krow = reinterpret_cast<uint32_t *>(kb.base + b_krow) + v * NS;
-        rc = run_scan(ctx, &qv, plan, slot, stream, kb.base + b_src, tlc, &out->base.stats, 0, true, &pass);
-        cudaError_t ce = cudaStreamSynchronize(stream);  // also on failure: nothing may be in flight when the slot goes back
-        if (!rc && ce != cudaSuccess) rc = fail(BYDB_EIO, cudaGetErrorString(ce));
-        if (!rc) rc = collect_scan(slot, &out->base.stats);
-        if (rc) return rc;
-    }
+    rc = keyed_passes(ctx, q, key, plan, slot, kv, kb.base + b_src, tlc, reinterpret_cast<int64_t *>(kb.base + b_ct),
+                      reinterpret_cast<int64_t *>(kb.base + b_kts), reinterpret_cast<uint32_t *>(kb.base + b_krow), &out->base.stats);
+    if (rc) return rc;
 
     // ---- 3. insertion order of the composite groups, table reordered, ordinary finalisation / Top-N on it
     KeyOrderParams ko;
@@ -1774,26 +1875,9 @@ int bydb_scan_agg_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key
     ko.n_groups = static_cast<int32_t>(G);
     ko.n_values = static_cast<uint32_t>(V);
     ko.n_series = static_cast<uint32_t>(NS);
-    // order | group_start of the series groups: rebuilt here (run_scan's copies live in its own scratch)
-    std::vector<int32_t> order(NS), gstart(G + 1, 0);
-    if (q->series_group) {
-        for (size_t i = 0; i < NS; ++i) gstart[static_cast<size_t>(q->series_group[i]) + 1]++;
-        for (size_t g = 0; g < G; ++g) gstart[g + 1] += gstart[g];
-        std::vector<int32_t> cur(gstart.begin(), gstart.end() - 1);
-        for (size_t i = 0; i < NS; ++i) order[cur[q->series_group[i]]++] = static_cast<int32_t>(i);
-    } else {
-        for (size_t i = 0; i < NS; ++i) order[i] = static_cast<int32_t>(i);
-        gstart[1] = static_cast<int32_t>(NS);
-    }
     Scratch kc;
-    kc.stream = stream;
-    const size_t c_order = 0, c_gstart = align_up(NS * 4, 256);
-    CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&kc.base), c_gstart + (G + 1) * 4, stream));
-    if (NS) memcpy(slot.pinned, order.data(), NS * 4);
-    memcpy(slot.pinned + c_gstart, gstart.data(), (G + 1) * 4);
-    CUDA_TRY(cudaMemcpyAsync(kc.base, slot.pinned, c_gstart + (G + 1) * 4, cudaMemcpyHostToDevice, stream));
-    ko.order = reinterpret_cast<const int32_t *>(kc.base + c_order);
-    ko.group_start = reinterpret_cast<const int32_t *>(kc.base + c_gstart);
+    rc = upload_group_order(q, G, slot, kc, &ko.order, &ko.group_start);
+    if (rc) return rc;
     ko.Kts = reinterpret_cast<const int64_t *>(kb.base + b_kts);
     ko.Krow = reinterpret_cast<const uint32_t *>(kb.base + b_krow);
     ko.slot = reinterpret_cast<int32_t *>(kb.base + b_slot);
@@ -1801,20 +1885,7 @@ int bydb_scan_agg_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key
     ko.perm = reinterpret_cast<int32_t *>(kb.base + b_perm);
     ko.n_present = reinterpret_cast<uint32_t *>(kb.base + b_np);
     launch_key_order(ko, stream);
-    auto table_ptrs = [&](uint8_t *t) {
-        TablePtrs tp;
-        tp.sum_f64 = reinterpret_cast<double *>(t + tlc.off_sum_f64);
-        tp.max_f64 = reinterpret_cast<double *>(t + tlc.off_max_f64);
-        tp.negmin_f64 = reinterpret_cast<double *>(t + tlc.off_negmin_f64);
-        tp.sum_i64 = reinterpret_cast<int64_t *>(t + tlc.off_sum_i64);
-        tp.cnt = reinterpret_cast<int64_t *>(t + tlc.off_cnt);
-        tp.rows = reinterpret_cast<int64_t *>(t + tlc.off_rows);
-        tp.max_i64 = reinterpret_cast<int64_t *>(t + tlc.off_max_i64);
-        tp.notmin_i64 = reinterpret_cast<int64_t *>(t + tlc.off_notmin_i64);
-        tp.coltype = reinterpret_cast<int64_t *>(t + tlc.off_coltype);
-        return tp;
-    };
-    launch_permute_table(table_ptrs(kb.base + b_dst), table_ptrs(kb.base + b_src), ko.perm, static_cast<uint32_t>(GP), static_cast<uint32_t>(F),
+    launch_permute_table(table_ptrs(kb.base + b_dst, tlc), table_ptrs(kb.base + b_src, tlc), ko.perm, static_cast<uint32_t>(GP), static_cast<uint32_t>(F),
                          reinterpret_cast<const int64_t *>(kb.base + b_ct), static_cast<uint32_t>(V), stream);
     CUDA_TRY(cudaStreamSynchronize(stream));  // the staging above is reused by the finalisation's read-back
     out->base.stats.kernel_launches += 3;
@@ -1829,15 +1900,7 @@ int bydb_scan_agg_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key
     CUDA_TRY(cudaMemcpyAsync(perm.data(), kb.base + b_perm, GP * 4, cudaMemcpyDeviceToHost, stream));
     CUDA_TRY(cudaStreamSynchronize(stream));
     out->base.stats.d2h_bytes += GP * 4;
-    // rows carry the position in insertion order: back to (group of the series, key value)
-    auto *ro = static_cast<ResultOwner *>(out->base.owner);
-    owner->key_id.resize(ro->group_id.size());
-    for (size_t r = 0; r < ro->group_id.size(); ++r) {
-        const int32_t comp = perm[static_cast<size_t>(ro->group_id[r])];
-        owner->key_id[r] = comp / static_cast<int32_t>(G);
-        ro->group_id[r] = comp % static_cast<int32_t>(G);
-    }
-    out->key_id = owner->key_id.data();
+    keyed_split_rows(out, perm, G);
     done = true;
     return 0;
     });
@@ -2878,6 +2941,296 @@ int bydb_scan_reduce(bydb_ctx *ctx, const bydb_query *q, int32_t root, bydb_resu
     if (!ctx || !out) return fail(BYDB_EINVAL, "ctx/out is NULL");
     memset(out, 0, sizeof *out);
     return scan_reduce_impl(ctx, q, nullptr, 0, 0, root, out);
+    });
+}
+
+// ------------------------------------------------------------------------------------------------
+// Keyed collective (bydb_scan_reduce_keyed): group-by on a stored tag over the peer mailboxes.  Each rank finds its own
+// distinct key values and runs one pass per value with its composite table landing straight in its slot of the root's
+// mailbox; the root unites the dictionaries, folds the slices through the remap and restores the single-context insertion
+// order (see "Keyed collective" in scan_kernels.cu).
+// ------------------------------------------------------------------------------------------------
+namespace {
+// One rank's slot, every piece 256-byte aligned:
+//   u32 V_r | u32 lens[cap] | bytes[cap x kMaxLit] (the rank's dictionary) | first appearance of composite group (v, g):
+//   u64 sid[cap x G], i64 Kts[cap x G], u32 Krow[cap x G] | i64 pass column types[cap x F] | composite table TableLayout(cap x G, F),
+//   value-major (slice v = groups v*G .. v*G + G - 1; only the first V_r slices are written)
+struct KeyedSlotLayout {
+    TableLayout tl;
+    size_t off_nv = 0, off_lens = 0, off_vals = 0, off_fsid = 0, off_fts = 0, off_frow = 0, off_ct = 0, off_table = 0, total = 0;
+    KeyedSlotLayout(size_t cap, size_t G, size_t F) : tl(cap * G, F) {
+        auto carve = [&](size_t bytes) {
+            const size_t at = total;
+            total = align_up(total + bytes, 256);
+            return at;
+        };
+        off_nv = carve(16);
+        off_lens = carve(cap * 4);
+        off_vals = carve(cap * kMaxLit);
+        off_fsid = carve(cap * G * 8);
+        off_fts = carve(cap * G * 8);
+        off_frow = carve(cap * G * 4);
+        off_ct = carve(cap * F * 8);
+        off_table = carve(tl.total);
+    }
+};
+}  // namespace
+
+int bydb_keyed_reduce_layout(const bydb_query *q, const bydb_group_key *key, uint64_t *slot_bytes) {
+    return guarded([&]() -> int {
+    if (!slot_bytes) return fail(BYDB_EINVAL, "slot_bytes is NULL");
+    int rc = validate_query(q, false);
+    if (rc) return rc;
+    if (!key || !key->family || !key->tag) return fail(BYDB_EINVAL, "group key without family/tag");
+    const uint32_t cap = key->max_values ? key->max_values : 64u;
+    if (cap > kMaxKeyValues) return fail(BYDB_EINVAL, "bydb_group_key.max_values above 256");
+    std::vector<std::string> fcols;
+    std::vector<int> agg_fcol;
+    distinct_fields(q, fcols, agg_fcol);
+    if (fcols.size() > kMaxFcols) return fail(BYDB_EINVAL, "too many distinct aggregated fields (max 8)");
+    const size_t G = q->series_group ? static_cast<size_t>(q->n_groups) : 1;
+    *slot_bytes = KeyedSlotLayout(cap, G, fcols.size()).total;
+    return 0;
+    });
+}
+
+int bydb_scan_reduce_keyed(bydb_ctx *ctx, const bydb_query *q, const bydb_group_key *key, int32_t root, bydb_keyed_result *out) {
+    return guarded([&]() -> int {
+    if (!ctx || !out) return fail(BYDB_EINVAL, "ctx/out is NULL");
+    memset(out, 0, sizeof *out);
+    Comm &cm = ctx->comm;
+    std::lock_guard<std::mutex> lk(cm.mu);
+    if (cm.nranks == 0) return fail(BYDB_EINVAL, "bydb_comm_connect was not called on this context");
+    if (root < 0 || root >= cm.nranks) return fail(BYDB_EINVAL, "bad root");
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    g_last_dev_err = 0;
+    SlotLease lease(ctx);
+    if (lease.init()) return fail(BYDB_EIO, "cannot create stream");
+    ExecSlot &es = *lease.slot;
+    cudaStream_t s = es.stream;
+    // From here on this rank ALWAYS raises its arrival flag with a status word in front of it (scan_reduce_impl's protocol): a
+    // failure on any rank reaches the root through the status words, and every rank counts the same epochs.
+    const uint64_t epoch = ++cm.epoch;
+    const size_t parity = static_cast<size_t>(epoch & 1u);
+    const size_t slot = cm.peer_slot_bytes[static_cast<size_t>(root)];
+    uint8_t *root_mb = cm.peer[static_cast<size_t>(root)];
+    uint8_t *slots0 = root_mb + kCommCtl + parity * static_cast<size_t>(cm.nranks) * slot;
+    uint8_t *my_slot = slots0 + static_cast<size_t>(cm.rank) * slot;
+    unsigned long long *flags = reinterpret_cast<unsigned long long *>(root_mb);
+    unsigned long long *status = reinterpret_cast<unsigned long long *>(root_mb + kCommStatusOff);
+    unsigned long long *done = reinterpret_cast<unsigned long long *>(root_mb + kCommDoneOff);
+    uint32_t *my_err = reinterpret_cast<uint32_t *>(cm.mine + kCommErrOff);
+    Plan plan;
+    uint32_t cap = 64;
+    int rc = keyed_prepare(ctx, q, key, plan, cap);
+    const size_t G = rc ? 1 : static_cast<size_t>(plan.n_groups), F = rc ? 1 : plan.fcols.size(), NS = rc ? 0 : q->n_series, A = rc ? 1 : q->n_aggs;
+    const KeyedSlotLayout kl(cap, G, F);
+    if (!rc && kl.total > slot) rc = fail(BYDB_EINVAL, "group-key table larger than the mailbox slots (size them with bydb_keyed_reduce_layout)");
+    if (!rc && cap * G > 0x7fffffffull / F) rc = fail(BYDB_ENOMEM, "group-key query: too many composite groups");
+    // the staging at its largest (the root's finalisation of up to cap x G groups) before any wait can spin (ExecSlot::ensure_pinned)
+    if (!rc && es.ensure_pinned(std::max(NS * 12 + (G + 1) * 4 + cap * G * (12 + 16 * A) + 16 * A + 8192, cap * (kMaxLit + 4) + NS * 8 + 4096)))
+        rc = fail(BYDB_ENOMEM, "cudaMallocHost failed");
+    memset(&out->base.stats, 0, sizeof out->base.stats);
+    bydb_stats &st = out->base.stats;
+    // the slots' previous use must have been consumed by the root before this rank writes into them
+    const uint64_t prev_use = cm.last_use[2 * static_cast<size_t>(root) + parity];
+    cm.last_use[2 * static_cast<size_t>(root) + parity] = epoch;
+    uint32_t host_perr = 0;
+    if (prev_use) {
+        if (cm.shared_device) host_perr = comm_wait_host(cm, done, 1, prev_use);
+        else launch_comm_wait(done, 1, prev_use, my_err, kErrPeerTimeout, s);
+    }
+    // map: distinct values, one pass per value into this rank's slot, the dictionary and the first appearances next to it
+    KeyValues kv;
+    Scratch kb, kc;
+    if (!rc) rc = [&]() -> int {
+        int r2 = keyed_values(ctx, q, key, cap, plan, es, &st, kv);
+        if (r2) return r2;
+        const size_t V = kv.values.size();
+        KeyFirstParams kf;
+        memset(&kf, 0, sizeof kf);
+        if (V) {
+            const size_t kts_bytes = align_up(V * NS * 8, 256);
+            kb.stream = s;
+            CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&kb.base), kts_bytes + V * NS * 4 + 256, s));
+            int64_t *kts = reinterpret_cast<int64_t *>(kb.base);
+            uint32_t *krow = reinterpret_cast<uint32_t *>(kb.base + kts_bytes);
+            CUDA_TRY(cudaMemsetAsync(my_slot + kl.off_ct, 0, V * F * 8, s));
+            r2 = keyed_passes(ctx, q, key, plan, es, kv, my_slot + kl.off_table, kl.tl, reinterpret_cast<int64_t *>(my_slot + kl.off_ct), kts, krow, &st);
+            if (r2) return r2;
+            r2 = upload_group_order(q, G, es, kc, &kf.order, &kf.group_start);
+            if (r2) return r2;
+            kf.Kts = kts;
+            kf.Krow = krow;
+        }
+        CUDA_TRY(cudaMemcpyAsync(my_slot + kl.off_lens, kv.d_lens, static_cast<size_t>(cap) * 4, cudaMemcpyDeviceToDevice, s));
+        CUDA_TRY(cudaMemcpyAsync(my_slot + kl.off_vals, kv.d_vals, static_cast<size_t>(cap) * kMaxLit, cudaMemcpyDeviceToDevice, s));
+        kf.n_groups = static_cast<int32_t>(G);
+        kf.n_values = static_cast<uint32_t>(V);
+        kf.q_sids = kv.d_sids;
+        kf.n_series = static_cast<uint32_t>(NS);
+        kf.n_values_out = reinterpret_cast<uint32_t *>(my_slot + kl.off_nv);
+        kf.first_sid = reinterpret_cast<uint64_t *>(my_slot + kl.off_fsid);
+        kf.first_ts = reinterpret_cast<int64_t *>(my_slot + kl.off_fts);
+        kf.first_row = reinterpret_cast<uint32_t *>(my_slot + kl.off_frow);
+        launch_key_first(kf, s);
+        st.kernel_launches += 1;
+        return 0;
+    }();
+    const std::string my_msg = rc ? g_last_error : std::string();
+    const unsigned long long st_word = (epoch << 32) | static_cast<unsigned long long>(static_cast<uint32_t>(-rc));
+    cudaMemcpyAsync(status + cm.rank, &st_word, sizeof st_word, cudaMemcpyHostToDevice, s);  // pageable source: staged before the call returns
+    launch_comm_signal(flags + cm.rank, epoch, s);
+    unsigned long long peer_status[kCommMaxRanks] = {0};
+    int frc = 0;
+    if (cm.rank == root) {
+        if (cm.shared_device) {
+            const uint32_t e2 = comm_wait_host(cm, flags, static_cast<uint32_t>(cm.nranks), epoch);
+            host_perr = host_perr ? host_perr : e2;
+        } else {
+            launch_comm_wait(flags, static_cast<uint32_t>(cm.nranks), epoch, my_err, kErrPeerTimeout, s);
+        }
+        cudaStreamSynchronize(s);
+        cudaMemcpy(peer_status, status, sizeof(unsigned long long) * static_cast<size_t>(cm.nranks), cudaMemcpyDeviceToHost);
+        uint32_t werr = 0;
+        cudaMemcpy(&werr, my_err, sizeof werr, cudaMemcpyDeviceToHost);
+        // reduce only over slots that every rank filled: a failed rank's slot holds nothing of this epoch
+        bool all_ok = !rc && !host_perr && !werr;
+        for (int r = 0; r < cm.nranks && all_ok; ++r)
+            all_ok = !((peer_status[r] >> 32) == (epoch & 0xffffffffull) && static_cast<uint32_t>(peer_status[r]) != 0);
+        if (all_ok) frc = [&]() -> int {
+            // 1. key union over the ranks' dictionaries
+            const size_t R = static_cast<size_t>(cm.nranks), n = R * cap;
+            size_t hash_slots = 64;
+            while (hash_slots < 2 * n) hash_slots <<= 1;
+            size_t o = 0;
+            auto carve = [&](size_t bytes) {
+                const size_t at = o;
+                o = align_up(o + bytes, 256);
+                return at;
+            };
+            const size_t u_hash = carve(hash_slots * 4), u_rep = carve(n * 4), u_remap = carve(n * 4), u_inv = carve(n * 4), u_ctl = carve(16),
+                         u_lens = carve(static_cast<size_t>(cap) * 4), u_vals = carve(static_cast<size_t>(cap) * kMaxLit);
+            Scratch ua;
+            ua.stream = s;
+            CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&ua.base), o, s));
+            CUDA_TRY(cudaMemsetAsync(ua.base + u_hash, 0, hash_slots * 4, s));
+            CUDA_TRY(cudaMemsetAsync(ua.base + u_remap, 0xff, u_ctl - u_remap, s));
+            CUDA_TRY(cudaMemsetAsync(ua.base + u_ctl, 0, o - u_ctl, s));
+            KeyUnionParams up;
+            memset(&up, 0, sizeof up);
+            up.n_ranks = static_cast<uint32_t>(R);
+            up.cap = cap;
+            up.slots = slots0;
+            up.slot_bytes = slot;
+            up.off_nv = kl.off_nv;
+            up.off_lens = kl.off_lens;
+            up.off_vals = kl.off_vals;
+            up.hash = reinterpret_cast<uint32_t *>(ua.base + u_hash);
+            up.hash_slots = static_cast<uint32_t>(hash_slots);
+            up.rep = reinterpret_cast<int32_t *>(ua.base + u_rep);
+            up.remap = reinterpret_cast<int32_t *>(ua.base + u_remap);
+            up.inv = reinterpret_cast<int32_t *>(ua.base + u_inv);
+            up.ctl = reinterpret_cast<uint32_t *>(ua.base + u_ctl);
+            up.g_lens = reinterpret_cast<uint32_t *>(ua.base + u_lens);
+            up.g_vals = ua.base + u_vals;
+            launch_key_union(up, s);
+            const size_t back = o - u_ctl;  // ctl | lens | vals
+            CUDA_TRY(cudaMemcpyAsync(es.pinned, ua.base + u_ctl, back, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(cudaStreamSynchronize(s));
+            CUDA_TRY(cudaGetLastError());
+            st.kernel_launches += 1;
+            st.d2h_bytes += back;
+            const uint32_t *ctl = reinterpret_cast<const uint32_t *>(es.pinned);
+            if (ctl[1] != 0) {
+                g_last_dev_err = ctl[1];
+                return fail(dev_err_code(ctl[1]), std::string(dev_err_text(ctl[1])) + " (the union of the ranks' values)");
+            }
+            const size_t Vg = ctl[0];
+            auto owner = new KeyedOwner();
+            out->owner = owner;
+            owner->key_off.push_back(0);
+            const uint32_t *hl = reinterpret_cast<const uint32_t *>(es.pinned + (u_lens - u_ctl));
+            const uint8_t *hv = es.pinned + (u_vals - u_ctl);
+            for (size_t v = 0; v < Vg; ++v) {
+                owner->key_bytes.insert(owner->key_bytes.end(), hv + v * kMaxLit, hv + v * kMaxLit + hl[v]);
+                owner->key_off.push_back(static_cast<uint32_t>(owner->key_bytes.size()));
+            }
+            if (owner->key_bytes.empty()) owner->key_bytes.push_back(0);
+            out->n_keys = static_cast<int32_t>(Vg);
+            out->key_off = owner->key_off.data();
+            out->key_bytes = owner->key_bytes.data();
+            if (Vg == 0) return 0;  // no rank selected a block: no rows
+            // 2. keyed combine, 3. order, then the single-context tail: permute, finalise, rows back to (series group, key)
+            const size_t GP = Vg * G;
+            const TableLayout tlc(GP, F);
+            o = 0;
+            const size_t c_comb = carve(tlc.total), c_dst = carve(tlc.total), c_ct = carve(Vg * F * 8), c_fsid = carve(GP * 8), c_fts = carve(GP * 8),
+                         c_frow = carve(GP * 4), c_perm = carve(GP * 4);
+            size_t sort_bytes = 0;
+            if (launch_key_rank(nullptr, nullptr, nullptr, nullptr, static_cast<uint32_t>(GP), nullptr, &sort_bytes, s))
+                return fail(BYDB_EIO, "cannot size the device sort of the composite groups");
+            const size_t c_sort = carve(sort_bytes);
+            Scratch ub;
+            ub.stream = s;
+            CUDA_TRY(cudaMallocAsync(reinterpret_cast<void **>(&ub.base), o, s));
+            KeyCombineParams cp;
+            memset(&cp, 0, sizeof cp);
+            cp.n_ranks = static_cast<uint32_t>(R);
+            cp.cap = cap;
+            cp.n_values = static_cast<uint32_t>(Vg);
+            cp.n_fcols = static_cast<uint32_t>(F);
+            cp.n_groups = static_cast<int32_t>(G);
+            cp.slot_bytes = slot;
+            cp.src = table_ptrs(slots0 + kl.off_table, kl.tl);
+            cp.src_ct = reinterpret_cast<const int64_t *>(slots0 + kl.off_ct);
+            cp.src_fsid = reinterpret_cast<const uint64_t *>(slots0 + kl.off_fsid);
+            cp.src_fts = reinterpret_cast<const int64_t *>(slots0 + kl.off_fts);
+            cp.src_frow = reinterpret_cast<const uint32_t *>(slots0 + kl.off_frow);
+            cp.inv = up.inv;
+            cp.dst = table_ptrs(ub.base + c_comb, tlc);
+            cp.dst_ct = reinterpret_cast<int64_t *>(ub.base + c_ct);
+            cp.fsid = reinterpret_cast<uint64_t *>(ub.base + c_fsid);
+            cp.fts = reinterpret_cast<int64_t *>(ub.base + c_fts);
+            cp.frow = reinterpret_cast<uint32_t *>(ub.base + c_frow);
+            launch_key_combine(cp, s);
+            int32_t *d_perm = reinterpret_cast<int32_t *>(ub.base + c_perm);
+            if (launch_key_rank(cp.fsid, cp.fts, cp.frow, d_perm, static_cast<uint32_t>(GP), ub.base + c_sort, &sort_bytes, s))
+                return fail(BYDB_EIO, "device sort of the composite groups failed");
+            launch_permute_table(table_ptrs(ub.base + c_dst, tlc), cp.dst, d_perm, static_cast<uint32_t>(GP), static_cast<uint32_t>(F), cp.dst_ct,
+                                 static_cast<uint32_t>(Vg), s);
+            st.kernel_launches += 4;  // combine, iota, the merge sort (counted once), permute
+            Plan planc = plan;
+            planc.n_groups = static_cast<int32_t>(GP);
+            int r2 = finalize_to_host(ctx, q, planc, es, s, ub.base + c_dst, tlc, &out->base, true);
+            if (r2) return r2;
+            std::vector<int32_t> perm(GP);
+            CUDA_TRY(cudaMemcpyAsync(perm.data(), d_perm, GP * 4, cudaMemcpyDeviceToHost, s));
+            CUDA_TRY(cudaStreamSynchronize(s));
+            st.d2h_bytes += GP * 4;
+            keyed_split_rows(out, perm, G);
+            return 0;
+        }();
+        cudaStreamSynchronize(s);
+        // the slots of this parity are free again: nothing reads them any more
+        cudaMemcpyAsync(done, &epoch, sizeof epoch, cudaMemcpyHostToDevice, s);
+    }
+    cudaStreamSynchronize(s);
+    uint32_t perr = 0;
+    if (cudaMemcpy(&perr, my_err, sizeof perr, cudaMemcpyDeviceToHost) == cudaSuccess && perr != 0) cudaMemset(my_err, 0, sizeof perr);
+    if (!perr) perr = host_perr;
+    // ---- outcome, most specific first: this rank's own failure, a failed wait, a peer's failure, the root's reduce
+    int crc = rc ? fail(rc, my_msg) : perr ? fail(dev_err_code(perr), dev_err_text(perr)) : 0;
+    if (!crc && cm.rank == root) {
+        for (int r = 0; r < cm.nranks && !crc; ++r) {
+            const unsigned long long w = peer_status[r];
+            if ((w >> 32) == (epoch & 0xffffffffull) && static_cast<uint32_t>(w) != 0)
+                crc = fail(-static_cast<int>(static_cast<uint32_t>(w)), "multi-GPU keyed reduce: rank " + std::to_string(r) + " failed");
+        }
+        if (!crc) crc = frc;
+    }
+    if (crc) bydb_keyed_result_free(ctx, out);
+    return crc;
     });
 }
 

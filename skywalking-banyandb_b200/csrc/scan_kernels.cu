@@ -19,6 +19,7 @@
 #include "lane_decode.cuh"
 
 #include <atomic>
+#include <cub/device/device_merge_sort.cuh>
 #include <cfloat>
 #include <cmath>
 #include <cstring>
@@ -3651,6 +3652,226 @@ void launch_permute_table(const TablePtrs &dst, const TablePtrs &src, const int3
     permute_table_kernel<<<(n + 255) / 256, 256, 0, s>>>(dst, src, perm, n_groups, n_fcols, pass_coltype, n_passes);
 }
 
+// ------------------------------------------------------------------------------------------------
+// Keyed collective (bydb_scan_reduce_keyed): group-by on a stored tag over the ranks' peer mailboxes.  Each rank finds ITS
+// distinct values and runs its per-value passes, so rank r's value v is not rank s's value v; what travels in the slot is
+// V_r, the rank's dictionary, the composite table and, per composite group, where it first showed (key_first_kernel).
+// The root then
+//   1. key_union_kernel: one CTA numbers the distinct values of all ranks in order of first occurrence over (rank, local id)
+//      -- a deterministic global dictionary -- and writes the remap (r, v) -> global id and its inverse;
+//   2. key_combine_kernel: folds the slices into one Vg x G table in rank order through the inverse (sums add, max / negmin
+//      take the maximum, the column types merge like permute_table's), and merges the first appearances (lexicographic
+//      minimum of (series id, Kts, Krow));
+//   3. launch_key_rank: sorts the composite groups by first appearance.  One context scanning everything inserts group (v, g)
+//      at (first series of g that shows v, rank of v among that series' first rows), and series ids ascend in the scan, so
+//      the sort gives the same insertion order; permute_table and the ordinary finalisation run on the result unchanged.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) key_first_kernel(const __grid_constant__ KeyFirstParams p) {
+    const int lane = threadIdx.x & 31;
+    const uint32_t gp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const uint32_t G = static_cast<uint32_t>(p.n_groups);
+    if (gp == 0 && lane == 0) *p.n_values_out = p.n_values;
+    if (gp >= G * p.n_values) return;
+    const uint32_t v = gp / G, g = gp % G;
+    const int64_t *kts = p.Kts + static_cast<size_t>(v) * p.n_series;
+    int32_t best = INT32_MAX;  // the query's series ascend: the smallest index is the smallest series id
+    for (int32_t k = p.group_start[g] + lane; k < p.group_start[g + 1]; k += 32) {
+        const int32_t i = p.order[k];
+        if (kts[i] != INT64_MAX && i < best) best = i;
+    }
+    best = __reduce_min_sync(0xffffffffu, best);
+    if (lane != 0) return;
+    if (best == INT32_MAX) {
+        p.first_sid[gp] = UINT64_MAX;
+        p.first_ts[gp] = INT64_MAX;
+        p.first_row[gp] = UINT32_MAX;
+    } else {
+        p.first_sid[gp] = p.q_sids[best];
+        p.first_ts[gp] = kts[best];
+        p.first_row[gp] = p.Krow[static_cast<size_t>(v) * p.n_series + best];
+    }
+}
+
+void launch_key_first(const KeyFirstParams &p, cudaStream_t s) {
+    const uint32_t n_comp = static_cast<uint32_t>(p.n_groups) * p.n_values;
+    key_first_kernel<<<n_comp ? (n_comp + 7) / 8 : 1, 256, 0, s>>>(p);
+}
+
+__global__ void __launch_bounds__(1024) key_union_kernel(const __grid_constant__ KeyUnionParams p) {
+    __shared__ uint32_t warp_tot[32];
+    const uint32_t n = p.n_ranks * p.cap, mask = p.hash_slots - 1;
+    // 1. every (rank, value) enters an open-addressing table keyed by its bytes (FNV-1a, as key_insert); the table keeps the
+    //    smallest entry index per distinct value.  rep[e] = the table slot for now.
+    for (uint32_t e = threadIdx.x; e < n; e += blockDim.x) {
+        const uint32_t r = e / p.cap, v = e % p.cap;
+        const uint8_t *slot = p.slots + static_cast<size_t>(r) * p.slot_bytes;
+        if (v >= *reinterpret_cast<const uint32_t *>(slot + p.off_nv)) {
+            p.rep[e] = -1;
+            continue;
+        }
+        const uint32_t len = reinterpret_cast<const uint32_t *>(slot + p.off_lens)[v];
+        const uint8_t *b = slot + p.off_vals + static_cast<size_t>(v) * kMaxLit;
+        uint64_t h = 0xcbf29ce484222325ull;
+        for (uint32_t i = 0; i < len; ++i) h = (h ^ b[i]) * 0x100000001b3ull;
+        uint32_t s = static_cast<uint32_t>(h ^ (h >> 32)) & mask;
+        for (;;) {  // hash_slots >= 2n: a free slot always exists
+            const uint32_t cur = atomicCAS(&p.hash[s], 0u, e + 1);
+            if (cur == 0) break;
+            const uint32_t o = cur - 1, ro = o / p.cap, vo = o % p.cap;
+            const uint8_t *so = p.slots + static_cast<size_t>(ro) * p.slot_bytes;
+            bool eq = reinterpret_cast<const uint32_t *>(so + p.off_lens)[vo] == len;
+            const uint8_t *bo = so + p.off_vals + static_cast<size_t>(vo) * kMaxLit;
+            for (uint32_t i = 0; i < len && eq; ++i) eq = bo[i] == b[i];
+            if (eq) {
+                atomicMin(&p.hash[s], e + 1);
+                break;
+            }
+            s = (s + 1) & mask;
+        }
+        p.rep[e] = static_cast<int32_t>(s);
+    }
+    __syncthreads();
+    // 2. the representative of an entry: the first (rank, value) with the same bytes
+    for (uint32_t e = threadIdx.x; e < n; e += blockDim.x)
+        if (p.rep[e] >= 0) p.rep[e] = static_cast<int32_t>(p.hash[p.rep[e]] - 1);
+    __syncthreads();
+    // 3. global ids: ordered compaction of the representatives over (rank, local id)
+    uint32_t base = 0;
+    for (uint32_t chunk = 0; chunk < n; chunk += blockDim.x) {
+        const uint32_t e = chunk + threadIdx.x;
+        const bool first = e < n && p.rep[e] == static_cast<int32_t>(e);
+        uint32_t total = 0;
+        const uint32_t pos = block_excl_scan(first ? 1u : 0u, warp_tot, total);
+        if (first) {
+            const uint32_t gid = base + pos, r = e / p.cap, v = e % p.cap;
+            p.remap[e] = static_cast<int32_t>(gid);
+            if (gid < p.cap) {
+                const uint8_t *slot = p.slots + static_cast<size_t>(r) * p.slot_bytes;
+                const uint32_t len = reinterpret_cast<const uint32_t *>(slot + p.off_lens)[v];
+                for (uint32_t i = 0; i < len; ++i) p.g_vals[static_cast<size_t>(gid) * kMaxLit + i] = slot[p.off_vals + static_cast<size_t>(v) * kMaxLit + i];
+                p.g_lens[gid] = len;
+                p.inv[r * p.cap + gid] = static_cast<int32_t>(v);
+            }
+        }
+        base += total;
+        __syncthreads();
+    }
+    // 4. every other entry takes the id of its representative
+    for (uint32_t e = threadIdx.x; e < n; e += blockDim.x) {
+        const int32_t rp = p.rep[e];
+        if (rp < 0 || rp == static_cast<int32_t>(e)) continue;
+        const int32_t gid = p.remap[rp];
+        p.remap[e] = gid;
+        if (static_cast<uint32_t>(gid) < p.cap) p.inv[(e / p.cap) * p.cap + static_cast<uint32_t>(gid)] = static_cast<int32_t>(e % p.cap);
+    }
+    if (threadIdx.x == 0) {
+        p.ctl[0] = base;
+        p.ctl[1] = base > p.cap ? static_cast<uint32_t>(kErrKeyCap) : 0u;
+    }
+}
+
+void launch_key_union(const KeyUnionParams &p, cudaStream_t s) { key_union_kernel<<<1, 1024, 0, s>>>(p); }
+
+template <class T>
+__device__ __forceinline__ const T *rank_ptr(const T *p0, uint32_t r, uint64_t stride) {
+    return reinterpret_cast<const T *>(reinterpret_cast<const uint8_t *>(p0) + r * stride);
+}
+
+// one thread per (composite group, field) of the Vg x G table
+__global__ void key_combine_kernel(const __grid_constant__ KeyCombineParams p) {
+    const uint32_t F = p.n_fcols, G = static_cast<uint32_t>(p.n_groups);
+    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= p.n_values * G * F) return;
+    const uint32_t j = t / F, c = t % F, vg = j / G, g = j % G;
+    double sf = 0, mf = 0, nf = 0;
+    int64_t si = 0, cn = 0, mi = 0, ni = 0, rows = 0;
+    uint64_t fsid = UINT64_MAX;
+    int64_t fts = INT64_MAX;
+    uint32_t frow = UINT32_MAX;
+    int64_t typ = 0, err = 0;
+    bool any = false;
+    for (uint32_t r = 0; r < p.n_ranks; ++r) {
+        const int32_t v = p.inv[r * p.cap + vg];
+        if (v < 0) continue;
+        const size_t sj = static_cast<size_t>(v) * G + g, so = sj * F + c;
+        const double bsf = rank_ptr(p.src.sum_f64, r, p.slot_bytes)[so], bmf = rank_ptr(p.src.max_f64, r, p.slot_bytes)[so],
+                     bnf = rank_ptr(p.src.negmin_f64, r, p.slot_bytes)[so];
+        const int64_t bsi = rank_ptr(p.src.sum_i64, r, p.slot_bytes)[so], bcn = rank_ptr(p.src.cnt, r, p.slot_bytes)[so],
+                      bmi = rank_ptr(p.src.max_i64, r, p.slot_bytes)[so], bni = rank_ptr(p.src.notmin_i64, r, p.slot_bytes)[so];
+        if (!any) {
+            sf = bsf, mf = bmf, nf = bnf, si = bsi, cn = bcn, mi = bmi, ni = bni;
+        } else {  // the rules of combine_tables_kernel
+            sf = sf + bsf;
+            mf = bmf > mf ? bmf : mf;
+            nf = bnf > nf ? bnf : nf;
+            si = static_cast<int64_t>(static_cast<uint64_t>(si) + static_cast<uint64_t>(bsi));  // wraps like Go's int64
+            cn += bcn;
+            mi = bmi > mi ? bmi : mi;
+            ni = bni > ni ? bni : ni;
+        }
+        if (c == 0) {
+            rows += rank_ptr(p.src.rows, r, p.slot_bytes)[sj];
+            const uint64_t s = rank_ptr(p.src_fsid, r, p.slot_bytes)[sj];
+            const int64_t ts = rank_ptr(p.src_fts, r, p.slot_bytes)[sj];
+            const uint32_t row = rank_ptr(p.src_frow, r, p.slot_bytes)[sj];
+            if (s < fsid || (s == fsid && (ts < fts || (ts == fts && row < frow)))) fsid = s, fts = ts, frow = row;
+        }
+        if (g == 0) {  // permute_table_kernel's merge of the passes' column types
+            const int64_t w = rank_ptr(p.src_ct, r, p.slot_bytes)[static_cast<size_t>(v) * F + c];
+            const int64_t wt = w & 0xff, we = w >> 8;
+            if (wt != 0 && typ != 0 && wt != typ) err = err > static_cast<int64_t>(kErrTypeMix) ? err : static_cast<int64_t>(kErrTypeMix);
+            if (typ == 0) typ = wt;
+            err = we > err ? we : err;
+        }
+        any = true;
+    }
+    p.dst.sum_f64[t] = sf;
+    p.dst.max_f64[t] = mf;
+    p.dst.negmin_f64[t] = nf;
+    p.dst.sum_i64[t] = si;
+    p.dst.cnt[t] = cn;
+    p.dst.max_i64[t] = mi;
+    p.dst.notmin_i64[t] = ni;
+    if (c == 0) {
+        p.dst.rows[j] = rows;
+        p.fsid[j] = fsid;
+        p.fts[j] = fts;
+        p.frow[j] = frow;
+    }
+    if (g == 0) p.dst_ct[static_cast<size_t>(vg) * F + c] = typ | (err << 8);
+}
+
+void launch_key_combine(const KeyCombineParams &p, cudaStream_t s) {
+    const uint32_t n = p.n_values * static_cast<uint32_t>(p.n_groups) * p.n_fcols;
+    if (n) key_combine_kernel<<<(n + 255) / 256, 256, 0, s>>>(p);
+}
+
+__global__ void iota_kernel(int32_t *out, uint32_t n) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = static_cast<int32_t>(i);
+}
+
+struct FirstAppearanceLess {
+    const uint64_t *sid;
+    const int64_t *ts;
+    const uint32_t *row;
+    __device__ bool operator()(int32_t a, int32_t b) const {
+        if (sid[a] != sid[b]) return sid[a] < sid[b];
+        if (ts[a] != ts[b]) return ts[a] < ts[b];
+        if (row[a] != row[b]) return row[a] < row[b];
+        return a < b;
+    }
+};
+
+int launch_key_rank(const uint64_t *fsid, const int64_t *fts, const uint32_t *frow, int32_t *perm, uint32_t n, void *temp, size_t *temp_bytes,
+                    cudaStream_t s) {
+    const FirstAppearanceLess less{fsid, fts, frow};
+    if (!temp) return cub::DeviceMergeSort::SortKeys(nullptr, *temp_bytes, perm, n, less, s) == cudaSuccess ? 0 : -1;
+    if (n == 0) return 0;
+    iota_kernel<<<(n + 255) / 256, 256, 0, s>>>(perm, n);
+    return cub::DeviceMergeSort::SortKeys(temp, *temp_bytes, perm, n, less, s) == cudaSuccess ? 0 : -1;
+}
+
 void launch_plan_blocks(const ScanParams &p, cudaStream_t s) {
     if (p.total_blocks == 0) return;
     const int threads = 256;
@@ -3840,6 +4061,10 @@ void preload_kernels() {
     (void)cudaFuncGetAttributes(&ka, key_order_kernel);
     (void)cudaFuncGetAttributes(&ka, key_perm_kernel);
     (void)cudaFuncGetAttributes(&ka, permute_table_kernel);
+    (void)cudaFuncGetAttributes(&ka, key_first_kernel);
+    (void)cudaFuncGetAttributes(&ka, key_union_kernel);
+    (void)cudaFuncGetAttributes(&ka, key_combine_kernel);
+    (void)cudaFuncGetAttributes(&ka, iota_kernel);
     cudaFuncAttributes a;
     cudaFuncGetAttributes(&a, plan_blocks_kernel);
     cudaFuncGetAttributes(&a, scan_blocks_kernel<true>);

@@ -223,6 +223,62 @@ struct TablePtrs {
 // dst[j] = src[perm[j]] for every group row of a partial table; coltype = the passes' column types merged
 void launch_permute_table(const TablePtrs &dst, const TablePtrs &src, const int32_t *perm, uint32_t n_groups, uint32_t n_fcols,
                           const int64_t *pass_coltype, uint32_t n_passes, cudaStream_t s);
+
+// ---- keyed collective (bydb_scan_reduce_keyed): see "Keyed collective" in scan_kernels.cu
+// every rank: where each composite group (v, g) first shows, as (series id, Kts, Krow); absent = (UINT64_MAX, INT64_MAX, UINT32_MAX)
+struct KeyFirstParams {
+    int32_t n_groups;
+    uint32_t n_values;
+    const uint64_t *q_sids;       // [n_series] ascending
+    const int32_t *order, *group_start;
+    const int64_t *Kts;           // [V * n_series]
+    const uint32_t *Krow;
+    uint32_t n_series;
+    uint32_t pad;
+    uint32_t *n_values_out;       // receives n_values (the rank's slot header)
+    uint64_t *first_sid;          // [V * G]
+    int64_t *first_ts;
+    uint32_t *first_row;
+};
+void launch_key_first(const KeyFirstParams &p, cudaStream_t s);
+// the root: the ranks' key dictionaries -> one global dictionary (ids in order of first occurrence over (rank, local id))
+struct KeyUnionParams {
+    uint32_t n_ranks, cap;        // every slot holds up to cap values
+    const uint8_t *slots;         // rank r's slot at slots + r * slot_bytes
+    uint64_t slot_bytes;
+    uint64_t off_nv, off_lens, off_vals;  // inside a slot: u32 V_r, u32 lens[cap], bytes[cap * kMaxLit]
+    uint32_t *hash;               // [hash_slots] zeroed: entry index + 1 of the first (rank, value) with those bytes
+    uint32_t hash_slots;          // power of two >= 2 * n_ranks * cap
+    int32_t *rep;                 // [n_ranks * cap] scratch
+    int32_t *remap;               // [n_ranks * cap] preset to -1: global id of (r, v)
+    int32_t *inv;                 // [n_ranks * cap] preset to -1: local id on rank r of global value g (index r * cap + g)
+    uint32_t *ctl;                // [0] distinct values over all ranks  [1] kErrKeyCap when that exceeds cap
+    uint32_t *g_lens;             // [cap] the global dictionary
+    uint8_t *g_vals;              // [cap * kMaxLit]
+};
+void launch_key_union(const KeyUnionParams &p, cudaStream_t s);
+// the root: the ranks' composite tables folded into one Vg x G table (rank order), first appearances merged
+struct KeyCombineParams {
+    uint32_t n_ranks, cap, n_values, n_fcols;  // n_values = Vg
+    int32_t n_groups;
+    uint32_t pad;
+    uint64_t slot_bytes;          // stride between the ranks' slots
+    TablePtrs src;                // composite table in rank 0's slot (cap * n_groups groups); rank r's is src + r * slot_bytes
+    const int64_t *src_ct;        // [cap * n_fcols] pass column types in rank 0's slot
+    const uint64_t *src_fsid;     // [cap * n_groups] first appearances in rank 0's slot
+    const int64_t *src_fts;
+    const uint32_t *src_frow;
+    const int32_t *inv;           // KeyUnionParams::inv
+    TablePtrs dst;                // Vg * n_groups groups
+    int64_t *dst_ct;              // [Vg * n_fcols] column types of the global values, merged over the ranks
+    uint64_t *fsid;               // [Vg * n_groups]
+    int64_t *fts;
+    uint32_t *frow;
+};
+void launch_key_combine(const KeyCombineParams &p, cudaStream_t s);
+// perm = 0..n-1 sorted by first appearance (sid, ts, row), absent groups last; temp == NULL: *temp_bytes receives the size
+int launch_key_rank(const uint64_t *fsid, const int64_t *fts, const uint32_t *frow, int32_t *perm, uint32_t n, void *temp, size_t *temp_bytes,
+                    cudaStream_t s);
 constexpr int kFusedFinalizeGroups = 8192;  // up to here one CTA finalises and selects in a single launch
 struct FinalizeParams;
 uint32_t launch_finalize_select(const FinalizeParams &fp, const SelectParams &p, cudaStream_t s);  // -> kernels launched
