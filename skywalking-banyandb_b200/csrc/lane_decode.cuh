@@ -166,6 +166,9 @@ BYDB_LANE_FN int32_t head_delta(uint32_t w0, uint32_t term, uint32_t prev_acc, u
 // class-0 part, so T0 / R0 hold twice their value (always even).  Lane result:
 //     T = T0/2 + 64*T1 + 8192*T2 = sum of the lane's byte contributions,  R' = same with weights rank+1,
 // page sum += (A + 1) * T - R'   with A = n - 1 - (terminators before the lane).
+// Class 2 only exists in varints of 3 or more bytes (|delta| >= 8192 units of the last decimal), which metric columns at a fixed
+// precision almost never hold: the scan runs the two-class form of the word (kTwoClass, five dot products) and decodes a chunk again
+// with the three-class form only when its guard says a class-2 byte is there.
 // ------------------------------------------------------------------------------------------------
 BYDB_LANE_FN uint32_t lane_prmt(uint32_t a, uint32_t b, uint32_t sel) {  // PTX prmt.b32, default mode (bit 3 of a selector nibble = replicate the byte's msb)
 #if defined(__CUDA_ARCH__)
@@ -218,37 +221,49 @@ BYDB_LANE_FN uint32_t mulhi_u32(uint32_t a, uint32_t b) {  // IMAD.HI: a right s
 
 struct SwarLane {
     int32_t T0, T1, T2, R0, R1, R2;
-    uint32_t wide;     // msb set in some byte <=> a varint of 4 or more bytes was seen
+    uint32_t wide;     // msb set in some byte <=> a varint of 4 or more bytes was seen (three-class words only)
+    uint32_t guard;    // msb set in some byte <=> the byte after it is of class 2 (two-class words only)
     int32_t nterm;     // 1 + terminators seen so far in this lane
     uint32_t prev_w;   // the word before the current one (the previous lane's last word for the first)
 };
 BYDB_LANE_FN void swar_begin(SwarLane &s, uint32_t prev_w) {
     s.T0 = s.T1 = s.T2 = s.R0 = s.R1 = s.R2 = 0;
-    s.wide = 0;
+    s.wide = s.guard = 0;
     s.nterm = 1;
     s.prev_w = prev_w;
 }
 // kMasked: first / last chunk of a page -- vm is 0xff for the bytes of the word that belong to the page; the others
 // neither terminate, nor carry payload, nor continue anything.
+// kTwoClass: the word as if no byte were of class 2 -- class 1 = every continued byte, its sign S1 -- which drops M2, S2, the
+// S12 select and the two class-2 dot products.  The guard collects w & M1 instead: an msb there = a continuation byte after
+// a continuation byte, so the NEXT byte is of class 2 (the third byte of a varint of 3 or more bytes) and the chunk has to be
+// decoded again by the three-class word.  Without class-2 bytes both forms give the same T, R' and terminator count, bit for bit.
 // Pipe balance (ncu r01: this integer kernel is bound by the ALU pipe, LOP3/PRMT/SHF, while the FMA pipe idles): everything
 // that can be a multiply-add is one -- the shifts by constants (IMAD / IMAD.HI), the in-word prefix sum, the running
 // terminator count (a dot product with 1s) and its broadcast.
-template <bool kMasked>
+template <bool kMasked, bool kTwoClass = false>
 BYDB_LANE_FN void swar_word(SwarLane &s, uint32_t w_in, uint32_t vm) {
     const uint32_t w = kMasked ? (w_in & vm) : w_in;
     const uint32_t pw = s.prev_w;
     const uint32_t p = w & 0x7f7f7f7fu;
     const uint32_t M1 = lane_prmt(w, pw, 0xA98Fu);   // byte i <- msb of byte i-1, replicated: 0xff = not the first byte of a varint
-    const uint32_t M2 = lane_prmt(w, pw, 0x98FEu);   // byte i <- msb of byte i-2
     const uint32_t sb = imad_u32(w, 128u, 0u);       // bit 0 of every byte moved to its msb (the low bits are don't-care)
     const uint32_t psb = imad_u32(pw, 128u, 0u);
     const uint32_t S0 = lane_prmt(sb, 0u, 0xBA98u);  // sign of a varint that starts at this byte
-    const uint32_t S1 = lane_prmt(sb, psb, 0xA98Fu); // ... that started one / two bytes earlier
-    const uint32_t S2 = lane_prmt(sb, psb, 0x98FEu);
-    const uint32_t S12 = (M2 & S2) | (~M2 & S1);     // sign of the varint a class-1 / class-2 byte belongs to
+    const uint32_t S1 = lane_prmt(sb, psb, 0xA98Fu); // ... that started one byte earlier
     const uint32_t x0 = (p ^ S0) & ~M1;              // class 0: int8 = 2 * (signed class-0 part); 0 elsewhere
-    const uint32_t p1 = p & M1 & ~M2;                // class 1 payloads
-    const uint32_t q2 = w & M1 & M2;                 // class 2 payloads; an msb here = a fourth byte follows (wide: the page bails out)
+    uint32_t p1, S12, q2 = 0;
+    if (kTwoClass) {
+        p1 = p & M1;                                 // class 1 payloads
+        S12 = S1;
+        s.guard |= w & M1;
+    } else {
+        const uint32_t M2 = lane_prmt(w, pw, 0x98FEu);    // byte i <- msb of byte i-2
+        const uint32_t S2 = lane_prmt(sb, psb, 0x98FEu);  // sign of a varint that started two bytes earlier
+        S12 = (M2 & S2) | (~M2 & S1);                     // sign of the varint a class-1 / class-2 byte belongs to
+        p1 = p & M1 & ~M2;                                // class 1 payloads
+        q2 = w & M1 & M2;                                 // class 2 payloads; an msb here = a fourth byte follows (wide: the page bails out)
+    }
     const uint32_t wT = S12 | 0x01010101u;           // +-1 (only read where p1 / q2 are non-zero, i.e. on class 1 / 2 bytes)
     uint32_t t01 = ~mulhi_u32(w, 1u << 25) & 0x01010101u;  // 1 where the byte terminates a varint
     if (kMasked) t01 &= vm;
@@ -261,11 +276,16 @@ BYDB_LANE_FN void swar_word(SwarLane &s, uint32_t w_in, uint32_t vm) {
     s.R0 = dp4a_su(x0, rank1, s.R0);
     s.T1 = dp4a_us(p1, wT, s.T1);
     s.R1 = dp4a_us(p1, wR, s.R1);
-    s.T2 = dp4a_us(q2, wT, s.T2);
-    s.R2 = dp4a_us(q2, wR, s.R2);
-    s.wide |= q2;
+    if (!kTwoClass) {
+        s.T2 = dp4a_us(q2, wT, s.T2);
+        s.R2 = dp4a_us(q2, wR, s.R2);
+        s.wide |= q2;
+    }
     s.prev_w = w;
 }
+// The word before a chunk ends in two continuation bytes: the chunk's first byte is of class 2, which the guard of the
+// chunk's own words cannot see (it lies behind the previous chunk's last byte).
+BYDB_LANE_FN bool swar_opens_class2(uint32_t last_w) { return ((last_w & (last_w << 8)) >> 31) != 0; }
 // -> number of terminators of the lane; T and R' as defined above
 BYDB_LANE_FN uint32_t swar_end(const SwarLane &s, int32_t &T, int32_t &Rp) {
     T = (s.T0 >> 1) + 64 * s.T1 + 8192 * s.T2;
@@ -354,35 +374,43 @@ BYDB_LANE_FN void swar_tail(uint32_t lw, uint32_t &accv, uint32_t &sh, int32_t &
 // ------------------------------------------------------------------------------------------------
 struct SwarMasked {
     int32_t T0, T1, T2, R0, R1, R2;
-    uint32_t wide;
+    uint32_t wide, guard;  // as in SwarLane
     int32_t nact;      // 1 + ACTIVE terminators seen so far in this lane
     uint32_t prev_w;
     uint32_t aw_lo, aw_hi;  // activity bits of the terminators still to come in this lane
 };
 BYDB_LANE_FN void swar_masked_begin(SwarMasked &s, uint32_t prev_w, uint32_t aw_lo, uint32_t aw_hi) {
     s.T0 = s.T1 = s.T2 = s.R0 = s.R1 = s.R2 = 0;
-    s.wide = 0;
+    s.wide = s.guard = 0;
     s.nact = 1;
     s.prev_w = prev_w;
     s.aw_lo = aw_lo;
     s.aw_hi = aw_hi;
 }
-template <bool kMasked>
+// kTwoClass: as in swar_word.
+template <bool kMasked, bool kTwoClass = false>
 BYDB_LANE_FN void swar_masked_word(SwarMasked &s, uint32_t w_in, uint32_t vm) {
     const uint32_t w = kMasked ? (w_in & vm) : w_in;
     const uint32_t pw = s.prev_w;
     const uint32_t p = w & 0x7f7f7f7fu;
     const uint32_t M1 = lane_prmt(w, pw, 0xA98Fu);
-    const uint32_t M2 = lane_prmt(w, pw, 0x98FEu);
     const uint32_t sb = imad_u32(w, 128u, 0u);
     const uint32_t psb = imad_u32(pw, 128u, 0u);
     const uint32_t S0 = lane_prmt(sb, 0u, 0xBA98u);
     const uint32_t S1 = lane_prmt(sb, psb, 0xA98Fu);
-    const uint32_t S2 = lane_prmt(sb, psb, 0x98FEu);
-    const uint32_t S12 = (M2 & S2) | (~M2 & S1);
     const uint32_t x0 = (p ^ S0) & ~M1;
-    const uint32_t p1 = p & M1 & ~M2;
-    const uint32_t q2 = w & M1 & M2;
+    uint32_t p1, S12, q2 = 0;
+    if (kTwoClass) {
+        p1 = p & M1;
+        S12 = S1;
+        s.guard |= w & M1;
+    } else {
+        const uint32_t M2 = lane_prmt(w, pw, 0x98FEu);
+        const uint32_t S2 = lane_prmt(sb, psb, 0x98FEu);
+        S12 = (M2 & S2) | (~M2 & S1);
+        p1 = p & M1 & ~M2;
+        q2 = w & M1 & M2;
+    }
     const uint32_t wT = S12 | 0x01010101u;
     uint32_t t01 = ~mulhi_u32(w, 1u << 25) & 0x01010101u;  // 1 where the byte terminates a varint
     if (kMasked) t01 &= vm;
@@ -406,9 +434,11 @@ BYDB_LANE_FN void swar_masked_word(SwarMasked &s, uint32_t w_in, uint32_t vm) {
     s.R0 = dp4a_su(x0, rank1, s.R0);
     s.T1 = dp4a_us(p1, wT, s.T1);
     s.R1 = dp4a_us(p1, wR, s.R1);
-    s.T2 = dp4a_us(q2, wT, s.T2);
-    s.R2 = dp4a_us(q2, wR, s.R2);
-    s.wide |= q2;
+    if (!kTwoClass) {
+        s.T2 = dp4a_us(q2, wT, s.T2);
+        s.R2 = dp4a_us(q2, wR, s.R2);
+        s.wide |= q2;
+    }
     s.prev_w = w;
 }
 // -> ACTIVE terminators of the lane; T and R' (active ranks)

@@ -691,7 +691,7 @@ __device__ __noinline__ int delta_page_fast(WarpSmem *sm, int lane) {
     return (row_base == count && carry_sh == 0) ? 0 : 2;
 }
 
-// One 1 KB chunk of a delta page through the SWAR lane decoder: loads the lane's 32 bytes from the staged tile, hands the
+// One 2 KB chunk of a delta page through the SWAR lane decoder: loads the lane's 64 bytes from the staged tile, hands the
 // neighbour's last word on, and returns the lane's terminator count n, its byte-linear sums T / R' and the wide flag.
 // c: chunk index inside the page window; carry_w: the (masked) last word of the previous chunk, updated.
 struct SwarChunk {
@@ -704,60 +704,71 @@ struct SwarChunk {
 constexpr uint32_t kSwarLaneBytes = 64;
 constexpr uint32_t kSwarChunkBytes = 32 * kSwarLaneBytes;
 static_assert(kStageBytes % kSwarChunkBytes == 0, "a TMA stage holds whole SWAR chunks");
+// The lane's 16 words through swar_word.  va / vb: valid bytes 0..31 / 32..63 of a first / last chunk of a page.  The
+// three-class pass only runs again over a chunk that holds a class-2 byte (rare), so it stays rolled to keep code small.
+template <bool kTwoClass>
+__device__ __forceinline__ void swar_chunk_pass(SwarLane &sl, const uint8_t *src, bool interior, uint32_t o, uint32_t total, uint32_t va, uint32_t vb,
+                                                uint32_t pw) {
+    swar_begin(sl, pw);
+    if (interior) {
+        // the two halves one after the other so that only 8 data words are live at a time
+#pragma unroll(kTwoClass ? 2 : 1)
+        for (int half = 0; half < 2; ++half) {
+            const uint4 wa = *reinterpret_cast<const uint4 *>(src + 32 * half), wb = *reinterpret_cast<const uint4 *>(src + 32 * half + 16);
+            swar_word<false, kTwoClass>(sl, wa.x, 0u);
+            swar_word<false, kTwoClass>(sl, wa.y, 0u);
+            swar_word<false, kTwoClass>(sl, wa.z, 0u);
+            swar_word<false, kTwoClass>(sl, wa.w, 0u);
+            swar_word<false, kTwoClass>(sl, wb.x, 0u);
+            swar_word<false, kTwoClass>(sl, wb.y, 0u);
+            swar_word<false, kTwoClass>(sl, wb.z, 0u);
+            swar_word<false, kTwoClass>(sl, wb.w, 0u);
+        }
+    } else {
+#pragma unroll(kTwoClass ? 4 : 1)
+        for (int q = 0; q < 4; ++q) {
+            uint4 w = make_uint4(0, 0, 0, 0);
+            if (o + 16 * q < total) w = *reinterpret_cast<const uint4 *>(src + 16 * q);
+            const uint32_t v = (q < 2 ? va : vb) >> (16 * (q & 1));
+            swar_word<true, kTwoClass>(sl, w.x, expand4(v));
+            swar_word<true, kTwoClass>(sl, w.y, expand4(v >> 4));
+            swar_word<true, kTwoClass>(sl, w.z, expand4(v >> 8));
+            swar_word<true, kTwoClass>(sl, w.w, expand4(v >> 12));
+        }
+    }
+}
+// The two-class pass first; when a byte of the chunk is of class 2 (a lane's guard, or the previous chunk ending in two
+// continuation bytes) the warp decodes the chunk again with the three-class word, which also raises `wide`.  Either way
+// n, T and R' are those of the three-class word.
 __device__ __forceinline__ SwarChunk swar_chunk(const uint8_t *buf, uint32_t c, uint32_t pstart, uint32_t pend, uint32_t total, uint32_t &carry_w, int lane) {
     const uint32_t o = c * kSwarChunkBytes + lane * kSwarLaneBytes;
     const bool interior = c * kSwarChunkBytes >= pstart && (c + 1) * kSwarChunkBytes <= pend;  // warp-uniform
     const uint8_t *src = buf + (o % kStageBytes);
-    SwarLane sl;
+    uint32_t va = 0xffffffffu, vb = 0xffffffffu, lastw;
     if (interior) {
-        // the neighbour only needs this lane's last word: fetch it first, then the two halves one after the other so that
-        // only 8 data words are live at a time
-        const uint32_t lastw = *reinterpret_cast<const uint32_t *>(src + kSwarLaneBytes - 4);
-        uint32_t pw = __shfl_up_sync(0xffffffffu, lastw, 1);
-        if (lane == 0) pw = carry_w;
-        carry_w = __shfl_sync(0xffffffffu, lastw, 31);
-        swar_begin(sl, pw);
-#pragma unroll
-        for (int half = 0; half < 2; ++half) {
-            const uint4 wa = *reinterpret_cast<const uint4 *>(src + 32 * half), wb = *reinterpret_cast<const uint4 *>(src + 32 * half + 16);
-            swar_word<false>(sl, wa.x, 0u);
-            swar_word<false>(sl, wa.y, 0u);
-            swar_word<false>(sl, wa.z, 0u);
-            swar_word<false>(sl, wa.w, 0u);
-            swar_word<false>(sl, wb.x, 0u);
-            swar_word<false>(sl, wb.y, 0u);
-            swar_word<false>(sl, wb.z, 0u);
-            swar_word<false>(sl, wb.w, 0u);
-        }
+        lastw = *reinterpret_cast<const uint32_t *>(src + kSwarLaneBytes - 4);
     } else {
-        uint4 w[4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            w[q] = make_uint4(0, 0, 0, 0);
-            if (o + 16 * q < total) w[q] = *reinterpret_cast<const uint4 *>(src + 16 * q);
-        }
         int lo_i = static_cast<int>(pstart) - static_cast<int>(o);
         int hi_i = static_cast<int>(pend) - static_cast<int>(o);
         lo_i = lo_i < 0 ? 0 : (lo_i > 64 ? 64 : lo_i);
         hi_i = hi_i < 0 ? 0 : (hi_i > 64 ? 64 : hi_i);
-        const uint32_t va = low_bits(hi_i > 32 ? 32 : hi_i) & ~low_bits(lo_i > 32 ? 32 : lo_i);               // bytes 0..31
-        const uint32_t vb = low_bits(hi_i > 32 ? hi_i - 32 : 0) & ~low_bits(lo_i > 32 ? lo_i - 32 : 0);       // bytes 32..63
-        const uint32_t mine = w[3].w & expand4(vb >> 28);
-        uint32_t pw = __shfl_up_sync(0xffffffffu, mine, 1);
-        if (lane == 0) pw = carry_w;
-        carry_w = __shfl_sync(0xffffffffu, mine, 31);
-        swar_begin(sl, pw);
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const uint32_t v = (q < 2 ? va : vb) >> (16 * (q & 1));
-            swar_word<true>(sl, w[q].x, expand4(v));
-            swar_word<true>(sl, w[q].y, expand4(v >> 4));
-            swar_word<true>(sl, w[q].z, expand4(v >> 8));
-            swar_word<true>(sl, w[q].w, expand4(v >> 12));
-        }
+        va = low_bits(hi_i > 32 ? 32 : hi_i) & ~low_bits(lo_i > 32 ? 32 : lo_i);               // bytes 0..31
+        vb = low_bits(hi_i > 32 ? hi_i - 32 : 0) & ~low_bits(lo_i > 32 ? lo_i - 32 : 0);       // bytes 32..63
+        lastw = o + 48 < total ? *reinterpret_cast<const uint32_t *>(src + kSwarLaneBytes - 4) & expand4(vb >> 28) : 0u;
     }
+    // the neighbour only needs this lane's last word: it is fetched first
+    uint32_t pw = __shfl_up_sync(0xffffffffu, lastw, 1);
+    const uint32_t cw = carry_w;
+    if (lane == 0) pw = cw;
+    carry_w = __shfl_sync(0xffffffffu, lastw, 31);
+    SwarLane sl;
+    swar_chunk_pass<true>(sl, src, interior, o, total, va, vb, pw);
     SwarChunk r;
-    r.wide = __any_sync(0xffffffffu, (sl.wide & 0x80808080u) != 0);
+    r.wide = false;
+    if (__any_sync(0xffffffffu, (sl.guard & 0x80808080u) != 0) || swar_opens_class2(cw)) {
+        swar_chunk_pass<false>(sl, src, interior, o, total, va, vb, pw);
+        r.wide = __any_sync(0xffffffffu, (sl.wide & 0x80808080u) != 0);
+    }
     r.n = swar_end(sl, r.T, r.Rp);
     return r;
 }
@@ -835,6 +846,34 @@ __device__ __noinline__ int delta_page_sum_all(WarpSmem *sm, int lane) {
 // rank taken over active terminators.  Lane contribution: ((A - a_0) - active terminators before the lane + 1) * T - R'.
 // One hot loop, like delta_page_sum_all.  Returns like delta_page_fast.
 // ------------------------------------------------------------------------------------------------
+// Pass 2 of delta_page_sum_masked over the lane's 16 words (va / vb: valid bytes 0..31 / 32..63 of a first / last chunk).
+template <bool kTwoClass>
+__device__ __forceinline__ void swar_masked_pass(SwarMasked &sl, const uint8_t *src, bool interior, uint32_t o, uint32_t total, uint32_t va, uint32_t vb,
+                                                 uint32_t pw, unsigned long long aw) {
+    swar_masked_begin(sl, pw, static_cast<uint32_t>(aw), static_cast<uint32_t>(aw >> 32));
+    if (interior) {
+#pragma unroll 1
+        for (int q = 0; q < 4; ++q) {
+            const uint4 w = *reinterpret_cast<const uint4 *>(src + 16 * q);
+            swar_masked_word<false, kTwoClass>(sl, w.x, 0u);
+            swar_masked_word<false, kTwoClass>(sl, w.y, 0u);
+            swar_masked_word<false, kTwoClass>(sl, w.z, 0u);
+            swar_masked_word<false, kTwoClass>(sl, w.w, 0u);
+        }
+    } else {
+#pragma unroll 1
+        for (int q = 0; q < 4; ++q) {
+            uint4 w = make_uint4(0, 0, 0, 0);
+            if (o + 16 * q < total) w = *reinterpret_cast<const uint4 *>(src + 16 * q);
+            const uint32_t v = (q < 2 ? va : vb) >> (16 * (q & 1));
+            swar_masked_word<true, kTwoClass>(sl, w.x, expand4(v));
+            swar_masked_word<true, kTwoClass>(sl, w.y, expand4(v >> 4));
+            swar_masked_word<true, kTwoClass>(sl, w.z, expand4(v >> 8));
+            swar_masked_word<true, kTwoClass>(sl, w.w, expand4(v >> 12));
+        }
+    }
+}
+
 template <int kMode>
 __device__ __noinline__ int delta_page_sum_masked(WarpSmem *sm, int lane) {
     static_assert(kMode != kRowsAll, "every row active: delta_page_sum_all");
@@ -912,37 +951,21 @@ __device__ __noinline__ int delta_page_sum_masked(WarpSmem *sm, int lane) {
             aw = (static_cast<unsigned long long>(__funnelshift_r(m1, m2, sft)) << 32 | __funnelshift_r(m0, m1, sft)) & nbits;
         }
         uint32_t pw = __shfl_up_sync(0xffffffffu, lastw, 1);
-        if (lane == 0) pw = carry_w;
+        const uint32_t cw = carry_w;
+        if (lane == 0) pw = cw;
         carry_w = __shfl_sync(0xffffffffu, lastw, 31);
-        // ---- pass 2: byte-linear sums, ranks over the active terminators
+        // ---- pass 2: byte-linear sums, ranks over the active terminators (two-class words; the three-class ones again over a
+        // chunk that holds a class-2 byte, as in swar_chunk)
         SwarMasked sl;
-        swar_masked_begin(sl, pw, static_cast<uint32_t>(aw), static_cast<uint32_t>(aw >> 32));
-        if (interior) {
-#pragma unroll 1
-            for (int q = 0; q < 4; ++q) {
-                const uint4 w = *reinterpret_cast<const uint4 *>(src + 16 * q);
-                swar_masked_word<false>(sl, w.x, 0u);
-                swar_masked_word<false>(sl, w.y, 0u);
-                swar_masked_word<false>(sl, w.z, 0u);
-                swar_masked_word<false>(sl, w.w, 0u);
+        swar_masked_pass<true>(sl, src, interior, o, st.total, va, vb, pw, aw);
+        if (__any_sync(0xffffffffu, (sl.guard & 0x80808080u) != 0) || swar_opens_class2(cw)) {
+            swar_masked_pass<false>(sl, src, interior, o, st.total, va, vb, pw, aw);
+            if (__any_sync(0xffffffffu, (sl.wide & 0x80808080u) != 0)) {
+                stream_drain(st, sm, k);
+                if (lane == 0) sm->seq = st.seq0 + min(st.nstages, k + static_cast<uint32_t>(kStages));
+                __syncwarp();
+                return 1;
             }
-        } else {
-#pragma unroll 1
-            for (int q = 0; q < 4; ++q) {
-                uint4 w = make_uint4(0, 0, 0, 0);
-                if (o + 16 * q < st.total) w = *reinterpret_cast<const uint4 *>(src + 16 * q);
-                const uint32_t v = (q < 2 ? va : vb) >> (16 * (q & 1));
-                swar_masked_word<true>(sl, w.x, expand4(v));
-                swar_masked_word<true>(sl, w.y, expand4(v >> 4));
-                swar_masked_word<true>(sl, w.z, expand4(v >> 8));
-                swar_masked_word<true>(sl, w.w, expand4(v >> 12));
-            }
-        }
-        if (__any_sync(0xffffffffu, (sl.wide & 0x80808080u) != 0)) {
-            stream_drain(st, sm, k);
-            if (lane == 0) sm->seq = st.seq0 + min(st.nstages, k + static_cast<uint32_t>(kStages));
-            __syncwarp();
-            return 1;
         }
         int32_t T, Rp;
         const uint32_t na = swar_masked_end(sl, T, Rp);
